@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — training images/sec of the fused LoRA step (BASELINE.json metric; default = configs[1], Qwen-Image-Edit).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME] [--dump-outputs DIR]
 
 --config  qwen_edit (default, BASELINE configs[1]) : Qwen-Image-Edit LoRA r=16 bf16, 512x512, cached embeds, batch 4 / GPU
           flux_kontext       (configs[2]) : FLUX-Kontext LoRA r=32 with the YAML target regex, 19+38 blocks, T=512, batch 2 / GPU
@@ -319,6 +319,30 @@ def library_baseline(dev, cfg, budget_s=150.0):
     return out
 
 
+DUMP_SAMPLE = 1 << 21  # elements kept of each flat LoRA array (fixed seeded positions): ~8 MB per array in float32
+
+
+def _step_outputs(m, loss, B):
+    """Host copies of what the last train_step handed its caller: the loss, the model's prediction over all image tokens, the summed
+    LoRA gradient and the LoRA parameters after the optimizer step.  The flat LoRA arrays (tens of millions of elements at full size)
+    are sampled at the same seeded positions every run, so two builds can be compared element for element."""
+    import torch
+
+    def sample(flat):
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+        return flat[idx.to(flat.device)].float().cpu()
+    params = torch.cat([p.detach().reshape(-1) for _, p in sorted(m._lora_params.items())])
+    return {"loss": loss.detach().float().reshape(1).cpu(), "pred": m._ws["pred"].view(B, -1, m._ws["pred"].shape[-1]).float().cpu(),
+            "lora_grad_sample": sample(m.G32), "lora_params_sample": sample(params)}
+
+
+def _dump_outputs(out_dir, outputs):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -383,6 +407,8 @@ def run_b200(args):
     e1.record()
     sync()
     launches = lib.LAUNCHES - n0
+    # snapshot of the last timed step, taken before the host-issue and e2e arms below run further optimizer steps
+    outputs = _step_outputs(m, loss, B) if args.dump_outputs and rank == 0 else None
     my_ms = e0.elapsed_time(e1) / args.steps
     ms = torch.tensor([my_ms], device=dev)
     per_rank = [my_ms]
@@ -476,6 +502,8 @@ def run_b200(args):
             "clocks": clk, "gpu_launches": launches, "host_issue_ms_per_step": host_issue_ms, "ms_per_step_per_rank": per_rank, "allreduce": allreduce,
             "e2e": {"value": e2e_ips, "unit": "images/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4},
             "roofline": roof, "cpu_baseline": cpu, "library_baseline": lib_base}
+    if outputs is not None:
+        _dump_outputs(args.dump_outputs, outputs)
     _emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -510,7 +538,13 @@ def main():
                     help="how a sharded block is assembled: copy-engine pulls from IPC-mapped peer shards (one node) or NCCL all-gather")
     ap.add_argument("--shard-weights", action="store_true",
                     help="frozen block weights sharded 1/N per rank, all-gathered per block (default for --config qwen_plus_sharded at N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss, prediction, sampled LoRA gradient and parameters) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:
